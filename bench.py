@@ -2,6 +2,7 @@
 """bench.py -- haystack GB/s of the batched Aho-Corasick search on B200 (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--config C2] [--impl ours|reference] [--mode strong|weak]
+                    [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one batch of synthetic haystacks.
 
@@ -22,6 +23,9 @@ A "step" is one pass of the hot path over one batch of synthetic haystacks.
   cpu_baseline  the reference's own C extension (oracle/_ref) looping iter() over the whole batch, single thread (the
             reference holds the GIL), rank 0 at N=1; its match list is compared with the GPU's (parity_checked)
   latency   microseconds per Automaton.iter() call on ONE haystack of 256 B / 64 KiB / 16 MiB, ours vs the reference
+
+--dump-outputs DIR writes what the last timed step returned (see dump_outputs) as DIR/<name>.npy, so that two builds can
+be compared output for output: the workload is generated from fixed seeds, identical from run to run.
 
 --impl reference times the reference extension on the host cores (one process per core, the pool created once, each
 worker looping iter() over its slice of a bounded sample) and prints the same JSON shape.
@@ -64,7 +68,11 @@ def parse():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-latency", action="store_true")
     ap.add_argument("--variant", default="planted", choices=["planted", "sparse"], help="sparse = pure random haystacks (diagnostic)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None, help="write the last timed step's match records to DIR/*.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 def default_scale(cfg, world):
@@ -273,6 +281,28 @@ def run_reference_arm(args):
 
 
 # --------------------------------------------------------------------------- our arm
+DUMP_LIMIT_BYTES = 64_000_000          # all files of one dump together, .npy headers included
+
+
+def dump_outputs(out_dir, d_out, n_matches, suffix=""):
+    """The records acb_scan_device() wrote (haystack, end_index, key_id), as float64 (exact for int32), in (haystack,
+    end_index, key_id) order: the kernels append them in whatever order their atomics give.  When the three columns
+    would pass DUMP_LIMIT_BYTES, a fixed seeded sample of the sorted rows is written instead (sample_rows.npy says
+    which); match_count.npy always holds the full count."""
+    rec = d_out[:n_matches].cpu().numpy().astype(np.int64)
+    rec = rec[np.lexsort((rec[:, 2], rec[:, 1], rec[:, 0]))]
+    os.makedirs(out_dir, exist_ok=True)
+    cols = {"hay_id": rec[:, 0], "end_index": rec[:, 1], "key_id": rec[:, 2]}
+    max_rows = (DUMP_LIMIT_BYTES - 4096) // (8 * (len(cols) + 1))
+    if n_matches > max_rows:
+        rows = np.sort(np.random.Generator(np.random.PCG64(0)).choice(n_matches, size=max_rows, replace=False))
+        cols = {k: v[rows] for k, v in cols.items()}
+        cols["sample_rows"] = rows
+    cols["match_count"] = np.array([n_matches])
+    for name, a in cols.items():
+        np.save(os.path.join(out_dir, f"{name}{suffix}.npy"), a.astype(np.float64))
+
+
 def latency_block(A, keys, sizes=(256, 65536, 16 * 1024 * 1024)):
     """microseconds per Automaton.iter() call (all matches drained) on ONE haystack, ours vs the reference extension"""
     import oracle
@@ -437,6 +467,11 @@ def main():
     barrier()
     ms_total = ev0.elapsed_time(ev1)
     kernel_ms = float(np.mean([a.elapsed_time(b) for a, b in kev]))
+    if args.dump_outputs:
+        last = int(d_cnt.item())
+        if last > cap:
+            raise SystemExit(f"rank {rank}: {last} matches do not fit the {cap}-record buffer, nothing to dump")
+        dump_outputs(args.dump_outputs, d_out, last, f"_rank{rank}" if world > 1 else "")
     launches = L.acb_launch_count() - launches0
     t = torch.tensor([ms_total], dtype=torch.float64, device="cuda")
     tot_bytes = torch.tensor([total], dtype=torch.int64, device="cuda")

@@ -1,13 +1,11 @@
 """Host-side API of the drop-in (everything that is not a search) compared call by call with the
-unmodified reference extension (oracle/_ref), both flavours.  CPU only; skipped where the reference
-extension did not travel."""
+unmodified reference extension, both flavours, as recorded in tests/golden/reference (tests/recorded_reference.py).
+CPU only."""
 import numpy as np
 import pytest
 
-import oracle
 import pyahocorasick_b200 as ac
-
-pytestmark = pytest.mark.skipif(not oracle.ref_available("bytes"), reason="oracle/_ref not built")
+from recorded_reference import reference  # noqa: F401 -- fixture
 
 
 def _conv(fl, s):
@@ -26,8 +24,8 @@ def _call(obj, name, *args):
 
 @pytest.mark.parametrize("fl", ["bytes", "unicode"])
 @pytest.mark.parametrize("seed", [1, 2, 3])
-def test_random_operation_sequences(fl, seed):
-    ref = oracle.ref_module(fl)
+def test_random_operation_sequences(fl, seed, reference):
+    ref = reference(fl)
     mine = ac.flavour(fl)
     rng = np.random.Generator(np.random.PCG64(seed))
     R, M = ref.Automaton(), mine.Automaton()
@@ -72,8 +70,8 @@ def test_random_operation_sequences(fl, seed):
 
 
 @pytest.mark.parametrize("fl", ["bytes", "unicode"])
-def test_wildcards_stores_and_errors(fl):
-    ref, mine = oracle.ref_module(fl), ac.flavour(fl)
+def test_wildcards_stores_and_errors(fl, reference):
+    ref, mine = reference(fl), ac.flavour(fl)
     c = lambda s: _conv(fl, s)  # noqa: E731
     R, M = ref.Automaton(), mine.Automaton()
     for i, w in enumerate(["he", "her", "hers", "she", "hi", "him", "his", "x", "h?r"]):
@@ -118,10 +116,10 @@ def test_wildcards_stores_and_errors(fl):
 
 
 @pytest.mark.parametrize("fl", ["bytes", "unicode"])
-def test_get_stats_counts_the_letter_trie_like_the_reference(fl):
+def test_get_stats_counts_the_letter_trie_like_the_reference(fl, reference):
     """nodes / links / words / longest_word of get_stats() (src/Automaton.c:1044-1097) after random add_word /
     remove_word / make_automaton / clear -- also for 4-byte letters, where the host arena holds one node per byte"""
-    ref, mod = oracle.ref_module(fl), ac.flavour(fl)
+    ref, mod = reference(fl), ac.flavour(fl)
     rng = np.random.default_rng(77)
     al = "ab\u0142\U0001f600" if fl == "unicode" else "abc"
 
@@ -162,13 +160,13 @@ def _mask_padding(chunks, letter_width):
 
 
 @pytest.mark.parametrize("fl", ["bytes", "unicode"])
-def test_enumeration_order_and_pickle_records_after_removals(fl):
+def test_enumeration_order_and_pickle_records_after_removals(fl, reference):
     """keys() / values() / items() in the reference's order (a pre-order walk that takes the most recently linked child
     first, src/AutomatonItemsIter.c:125-288) and __reduce__ records identical to the reference's (pre-order, children in
     link order, src/trie.c:197-213) -- also after remove_word and re-adding, when a re-made link goes to the END of its
     parent's child array in the reference (src/trie.c:66-136, src/trienode.c:125-147)"""
     from pyahocorasick_b200 import serialize
-    ref, mod = oracle.ref_module(fl), ac.flavour(fl)
+    ref, mod = reference(fl), ac.flavour(fl)
     rng = np.random.default_rng(2026)
     al = "ab\u0142\U0001f600" if fl == "unicode" else "abcd"
     for trial in range(150):

@@ -3,7 +3,7 @@
 Bar: bit-exact records (integer/index work).  Sources of truth, in order:
   1. tests/golden/*.json  -- produced by the unmodified reference (both flavours);
   2. oracle.OracleAutomaton -- the pinned C restatement, on seeded random batches at sizes it
-     finishes in seconds; the compiled reference (oracle/_ref) too when it travelled along;
+     finishes in seconds; the compiled reference too, as recorded in tests/golden/reference;
   3. at BASELINE.json's full sizes: properties that need no CPU run -- every planted
      occurrence is reported, no duplicates, each reported record really is an occurrence
      (sampled), and the two independent kernels (filter / DFA) agree exactly.
@@ -16,6 +16,7 @@ import pyahocorasick_b200 as ac
 from golden_driver import all_scenarios, run_ops
 from pyahocorasick_b200 import automaton as am
 from pyahocorasick_b200 import synth
+from recorded_reference import reference_records  # noqa: F401 -- fixture
 
 pytestmark = pytest.mark.gpu
 B = ac.flavour("bytes")
@@ -97,17 +98,21 @@ def test_random_batches_match_oracle(case, algo):
     assert _records(A.find_all_batch(hs, algo=algo)) == want3
 
 
-@pytest.mark.skipif(not oracle.ref_available("bytes"), reason="oracle/_ref did not travel")
-def test_reference_extension_agrees_on_c2_sample():
-    """The unmodified reference (compiled into oracle/_ref) on a C2 sub-sample."""
-    ref = oracle.ref_module("bytes")
+def _reference_batch(keys, rows):
+    def compute(ref):
+        R = ref.Automaton(ref.STORE_INTS)
+        for i, k in enumerate(keys):
+            R.add_word(k, i)
+        R.make_automaton()
+        return oracle.ref_scan_batch(R, [row.tobytes() for row in rows])
+    return compute
+
+
+def test_reference_extension_agrees_on_c2_sample(reference_records):
+    """The unmodified reference on a C2 sub-sample."""
     w = synth.make("C2", scale=0.005)
-    R = ref.Automaton(ref.STORE_INTS)
-    for i, k in enumerate(w.keys):
-        R.add_word(k, i)
-    R.make_automaton()
     A = synth.build_automaton(w.keys)
-    want = oracle.ref_scan_batch(R, [row.tobytes() for row in w.haystacks])
+    want = reference_records("c2_sample", _reference_batch(w.keys, w.haystacks))
     for algo in ("filter", "dfa"):
         m = A.find_all_batch(w.haystacks, algo=algo)
         assert list(zip(m.hay_id.tolist(), m.end_index.tolist(), m.values())) == want
@@ -231,37 +236,30 @@ def _check_full(w, A, sample=20000):
     return len(got)
 
 
-def _check_reference_rows(w, A, rows):
-    """the compiled reference (oracle/_ref) over the listed haystacks: identical records in identical order"""
-    if not oracle.ref_available("bytes"):
-        pytest.skip("oracle/_ref did not travel")
-    ref = oracle.ref_module("bytes")
-    R = ref.Automaton(ref.STORE_INTS)
-    for i, k in enumerate(w.keys):
-        R.add_word(k, i)
-    R.make_automaton()
+def _check_reference_rows(w, A, rows, reference_records):
+    """the compiled reference over the listed haystacks: identical records in identical order"""
     sub = np.ascontiguousarray(w.haystacks[rows])
-    want = [(h, e, v) for h in range(len(rows)) for e, v in R.iter(sub[h].tobytes())]
+    want = reference_records("rows", _reference_batch(w.keys, sub))
     m = A.find_all_batch(sub)
     assert list(zip(m.hay_id.tolist(), m.end_index.tolist(), m.values())) == want
 
 
-def test_full_size_c2_properties():
+def test_full_size_c2_properties(reference_records):
     w = synth.make("C2", scale=1.0)
     A = synth.build_automaton(w.keys)
     n = _check_full(w, A)
     assert n >= w.n_hay
-    _check_reference_rows(w, A, np.arange(0, w.n_hay, 10))           # every 10th haystack: 100 k, BASELINE.md section 2
+    _check_reference_rows(w, A, np.arange(0, w.n_hay, 10), reference_records)   # every 10th haystack: 100 k, BASELINE.md section 2
 
 
-def test_full_size_c3_dna_properties():
+def test_full_size_c3_dna_properties(reference_records):
     w = synth.make("C3", scale=1.0)          # BASELINE config 3 at its stated size: 10 M reads x 150 B, 100 k 20-mers
     A = synth.build_automaton(w.keys)
     _check_full(w, A)
-    _check_reference_rows(w, A, np.arange(0, w.n_hay, 100))          # 100 k reads through the reference
+    _check_reference_rows(w, A, np.arange(0, w.n_hay, 100), reference_records)  # 100 k reads through the reference
 
 
-def test_full_size_c4_long_haystacks_properties():
+def test_full_size_c4_long_haystacks_properties(reference_records):
     w = synth.make("C4", scale=1.0)          # BASELINE config 4 at its stated size: 64 x 16 MiB, a key across every 16 KiB
     A = synth.build_automaton(w.keys)
     # more straddlers, one across every boundary the kernel or the host pipeline has: 512-byte slices of a tile, the
@@ -293,14 +291,14 @@ def test_full_size_c4_long_haystacks_properties():
     w.planted_hay, w.planted_end, w.planted_key = ph[ok], pe[ok], pk[ok]
     assert len(extra_h) > 40
     _check_full(w, A)
-    _check_reference_rows(w, A, np.array([1]))                        # one whole 16 MiB haystack through the reference
+    _check_reference_rows(w, A, np.array([1]), reference_records)     # one whole 16 MiB haystack through the reference
 
 
-def test_c5_100k_keys_properties():
+def test_c5_100k_keys_properties(reference_records):
     w = synth.make("C5", scale=0.125)        # 1 M x 256 B (one GPU's shard of BASELINE config 5), 100 k keys
     A = synth.build_automaton(w.keys)
     _check_full(w, A)
-    _check_reference_rows(w, A, np.arange(0, w.n_hay, 10))
+    _check_reference_rows(w, A, np.arange(0, w.n_hay, 10), reference_records)
 
 
 def test_dense_matches_grow_the_buffers():

@@ -1,4 +1,4 @@
-"""AutomatonSearchIterLong.set() (src/AutomatonSearchIterLong.c:156-212) against the reference extension:
+"""AutomatonSearchIterLong.set() (src/AutomatonSearchIterLong.c:156-212) against the reference extension (as recorded):
 random keys, random chunks, set() after a random number of next() calls (before a match, between matches,
 after exhaustion, after extra calls past exhaustion), with and without reset.  On CPU the device is the
 emulation of tests/emul.py; the gpu-marked twin runs the real ACB_ALGO_LONG kernel."""
@@ -6,14 +6,11 @@ import numpy as np
 import pytest
 
 import emul
-import oracle
 import pyahocorasick_b200 as pkg
+from recorded_reference import reference  # noqa: F401 -- fixture
 
-needs_ref = pytest.mark.skipif(not oracle.ref_available("bytes"), reason="needs oracle/_ref")
-
-
-def _fuzz(fl, trials, seed):
-    ref, mod = oracle.ref_module(fl), pkg.flavour(fl)
+def _fuzz(ref, fl, trials, seed):
+    mod = pkg.flavour(fl)
     rng = np.random.default_rng(seed)
     al = "abc"
 
@@ -22,7 +19,7 @@ def _fuzz(fl, trials, seed):
         return s.encode() if fl == "bytes" else s
 
     for _ in range(trials):
-        keys = list({word(1, 5) for _ in range(int(rng.integers(1, 8)))})
+        keys = list(dict.fromkeys(word(1, 5) for _ in range(int(rng.integers(1, 8)))))
         A, R = mod.Automaton(), ref.Automaton()
         for i, k in enumerate(keys):
             A.add_word(k, i), R.add_word(k, i)
@@ -46,18 +43,16 @@ def _fuzz(fl, trials, seed):
         assert got == want, (fl, keys, chunks)
 
 
-@needs_ref
 @pytest.mark.parametrize("fl", ["bytes", "unicode"])
-def test_iter_long_set_matches_the_reference_emulated(fl, monkeypatch):
+def test_iter_long_set_matches_the_reference_emulated(fl, monkeypatch, reference):
     emul.install(monkeypatch, "filter")
-    _fuzz(fl, 150, 11)
+    _fuzz(reference(fl), fl, 150, 11)
 
 
-@needs_ref
 @pytest.mark.gpu
 @pytest.mark.parametrize("fl", ["bytes", "unicode"])
-def test_iter_long_set_matches_the_reference_on_gpu(fl):
-    _fuzz(fl, 25, 12)
+def test_iter_long_set_matches_the_reference_on_gpu(fl, reference):
+    _fuzz(reference(fl), fl, 25, 12)
 
 
 def test_iter_long_set_documented_example_and_errors(monkeypatch):
@@ -126,11 +121,10 @@ def test_iter_long_stream_uploads_only_the_new_chunk(monkeypatch):
     assert sizes[-5:] == [1] * 5
 
 
-@needs_ref
 @pytest.mark.gpu
-def test_iter_long_long_stream_on_gpu():
+def test_iter_long_long_stream_on_gpu(reference):
     """the same stream through the real ACB_ALGO_LONG kernel, against the reference extension"""
-    ref, mod = oracle.ref_module("bytes"), pkg.flavour("bytes")
+    ref, mod = reference("bytes"), pkg.flavour("bytes")
     A, R = _stream_case(mod), _stream_case(ref)
     rng = np.random.default_rng(5)
     ia, ir = A.iter_long(b"z" * 100), R.iter_long(b"z" * 100)

@@ -1,13 +1,14 @@
 """Pin the CPU oracle (oracle/ac_oracle.c) before anything trusts it.
 
 1. against the committed golden vectors (produced by the reference itself),
-2. against the compiled reference (oracle/_ref) on seeded random batches, when present.
+2. against the compiled reference on seeded random batches, as recorded in tests/golden/reference.
 """
 import numpy as np
 import pytest
 
 import oracle
 from golden_driver import all_scenarios, dec
+from recorded_reference import reference, reference_records  # noqa: F401 -- fixtures
 
 STORE_INTS, STORE_LENGTH, STORE_ANY = 10, 20, 30
 
@@ -108,26 +109,28 @@ def test_oracle_matches_golden(sc):
     assert checked or not sc.get("make", True) or not sc["words"]
 
 
-@pytest.mark.skipif(not oracle.ref_available("bytes"), reason="oracle/_ref not built")
+def _int_automaton(mod, keys):
+    A = mod.Automaton(mod.STORE_INTS)
+    for i, k in enumerate(keys):
+        A.add_word(k, i)
+    A.make_automaton()
+    return A
+
+
 @pytest.mark.parametrize("seed,alpha,nw,lens,nh,hl", [
     (1, b"ab", 30, (1, 8), 50, 300),
     (2, b"ACGT", 2000, (8, 12), 200, 150),
     (3, bytes(range(48, 58)) + bytes(range(65, 91)) + bytes(range(97, 123)), 1000, (4, 16), 400, 256),
     (4, bytes(range(256)), 500, (1, 4), 100, 1000),
 ])
-def test_oracle_matches_reference_batch(seed, alpha, nw, lens, nh, hl):
-    ref = oracle.ref_module("bytes")
+def test_oracle_matches_reference_batch(seed, alpha, nw, lens, nh, hl, reference, reference_records):
     rng = np.random.Generator(np.random.PCG64(seed))
     al = np.frombuffer(alpha, dtype=np.uint8)
-    R = ref.Automaton(ref.STORE_INTS)
+    keys = [al[rng.integers(0, len(al), size=int(rng.integers(lens[0], lens[1] + 1)))].tobytes() for _ in range(nw)]
+    R = _int_automaton(reference("bytes"), keys)
     O = oracle.OracleAutomaton()
-    keys = []
-    for i in range(nw):
-        k = al[rng.integers(0, len(al), size=int(rng.integers(lens[0], lens[1] + 1)))].tobytes()
-        keys.append(k)
-        R.add_word(k, i)
+    for i, k in enumerate(keys):
         O.add_word(k, i)
-    R.make_automaton()
     O.make_automaton()
     assert len(R) == len(O)
     assert R.get_stats()["nodes_count"] == O.nodes_count
@@ -138,6 +141,7 @@ def test_oracle_matches_reference_batch(seed, alpha, nw, lens, nh, hl):
         flat[h * hl + p:h * hl + p + len(k)] = k
     off = np.arange(nh + 1, dtype=np.int64) * hl
     got = O.scan_batch_bytes(flat, off)
-    want = oracle.ref_scan_batch(R, [flat[off[h]:off[h + 1]].tobytes() for h in range(nh)])
-    assert len(want) > 0
+    hays = [flat[off[h]:off[h + 1]].tobytes() for h in range(nh)]
+    want = reference_records("batch", lambda ref: oracle.ref_scan_batch(_int_automaton(ref, keys), hays))
+    assert want.n > 0
     assert [tuple(r) for r in got.tolist()] == want      # same records, same order

@@ -1,4 +1,4 @@
-"""iter() / find_all() argument handling against the reference extension, randomised: start / end (negative too),
+"""iter() / find_all() argument handling against the reference extension (as recorded in tests/golden/reference), randomised: start / end (negative too),
 ignore_white_space, find_all's callback form, chunked iteration with set() at random points.  The device is
 the CPU emulation (tests/emul.py); what is under test is the host layer's index arithmetic and state carry-over
 (src/Automaton.c:875-966, src/utils.c:293-359, src/AutomatonSearchIter.c:243-368)."""
@@ -8,19 +8,17 @@ import pytest
 import emul
 import oracle
 import pyahocorasick_b200 as pkg
+from recorded_reference import reference  # noqa: F401 -- fixture
 
-needs_ref = pytest.mark.skipif(not oracle.ref_available("bytes"), reason="needs oracle/_ref")
-
-
-def _pair(fl, rng, with_space):
-    ref, mod = oracle.ref_module(fl), pkg.flavour(fl)
+def _pair(ref, fl, rng, with_space):
+    mod = pkg.flavour(fl)
     al = "abc " if with_space else "abc"
 
     def word(lo, hi, alphabet=al):
         s = "".join(alphabet[int(j)] for j in rng.integers(0, len(alphabet), size=int(rng.integers(lo, hi))))
         return s.encode() if fl == "bytes" else s
 
-    keys = list({word(1, 5, "abc") for _ in range(int(rng.integers(1, 9)))})
+    keys = list(dict.fromkeys(word(1, 5, "abc") for _ in range(int(rng.integers(1, 9)))))
     A, R = mod.Automaton(), ref.Automaton()
     for i, k in enumerate(keys):
         A.add_word(k, i), R.add_word(k, i)
@@ -35,13 +33,12 @@ def _call(fn, *a, **kw):
         return ("exc", type(e).__name__)
 
 
-@needs_ref
 @pytest.mark.parametrize("fl", ["bytes", "unicode"])
-def test_iter_ranges_and_white_space(fl, monkeypatch):
+def test_iter_ranges_and_white_space(fl, monkeypatch, reference):
     emul.install(monkeypatch, "filter")
     rng = np.random.default_rng(21)
     for _ in range(120):
-        A, R, word = _pair(fl, rng, with_space=True)
+        A, R, word = _pair(reference(fl), fl, rng, with_space=True)
         hay = word(0, 30)
         n = len(hay)
         for _ in range(6):
@@ -56,13 +53,12 @@ def test_iter_ranges_and_white_space(fl, monkeypatch):
             assert _call(A.iter, *args, **kw) == _call(R.iter, *args, **kw), (fl, hay, args, kw)
 
 
-@needs_ref
 @pytest.mark.parametrize("fl", ["bytes", "unicode"])
-def test_find_all_ranges(fl, monkeypatch):
+def test_find_all_ranges(fl, monkeypatch, reference):
     emul.install(monkeypatch, "filter")
     rng = np.random.default_rng(22)
     for _ in range(100):
-        A, R, word = _pair(fl, rng, with_space=False)
+        A, R, word = _pair(reference(fl), fl, rng, with_space=False)
         hay = word(0, 30)
         n = len(hay)
         for _ in range(5):
@@ -82,17 +78,16 @@ def test_find_all_ranges(fl, monkeypatch):
             assert (run(A, got), got) == (run(R, want), want), (fl, hay, extra)
 
 
-@needs_ref
 @pytest.mark.parametrize("ws", [False, True])
 @pytest.mark.parametrize("fl", ["bytes", "unicode"])
-def test_iter_set_at_random_points(fl, ws, monkeypatch):
+def test_iter_set_at_random_points(fl, ws, monkeypatch, reference):
     """chunks shorter than the longest key (the history then holds everything seen so far), empty chunks, extra
     next() calls past exhaustion (each moves the reference's index on by one), reset, ignore_white_space"""
     emul.install(monkeypatch, "filter")
     rng = np.random.default_rng(23 + ws)
     kw = {"ignore_white_space": True} if ws else {}
     for _ in range(150):
-        A, R, word = _pair(fl, rng, with_space=ws)
+        A, R, word = _pair(reference(fl), fl, rng, with_space=ws)
         chunks = [word(0, 14) for _ in range(4)]
         ia, ir = A.iter(chunks[0], **kw), R.iter(chunks[0], **kw)
         got, want = [], []
@@ -112,12 +107,11 @@ def test_iter_set_at_random_points(fl, ws, monkeypatch):
         assert got == want, (fl, chunks)
 
 
-@needs_ref
 @pytest.mark.parametrize("fl", ["bytes", "unicode"])
-def test_batch_input_forms_equal_looping_the_reference(fl, monkeypatch):
+def test_batch_input_forms_equal_looping_the_reference(fl, monkeypatch, reference):
     """find_all_batch over a list, over (flat, offsets), over a uint8 matrix == iter() of the reference per haystack"""
     emul.install(monkeypatch, "filter")
-    ref, mod = oracle.ref_module(fl), pkg.flavour(fl)
+    ref, mod = reference(fl), pkg.flavour(fl)
     rng = np.random.default_rng(31)
     al = "ab\u0142" if fl == "unicode" else "abc"
 
@@ -126,7 +120,7 @@ def test_batch_input_forms_equal_looping_the_reference(fl, monkeypatch):
         return s.encode() if fl == "bytes" else s
 
     for _ in range(60):
-        keys = list({word(1, 6) for _ in range(int(rng.integers(1, 8)))})
+        keys = list(dict.fromkeys(word(1, 6) for _ in range(int(rng.integers(1, 8)))))
         A, R = mod.Automaton(), ref.Automaton()
         for i, k in enumerate(keys):
             A.add_word(k, (i, k)), R.add_word(k, (i, k))
@@ -144,11 +138,10 @@ def test_batch_input_forms_equal_looping_the_reference(fl, monkeypatch):
             assert list(A.find_all_batch(rows)) == [(h, e, v) for h in range(rows.shape[0]) for e, v in R.iter(rows[h].tobytes())]
 
 
-@needs_ref
 @pytest.mark.parametrize("fl", ["bytes", "unicode"])
-def test_key_sequences_iter_and_iter_long(fl, monkeypatch):
+def test_key_sequences_iter_and_iter_long(fl, monkeypatch, reference):
     emul.install(monkeypatch, "filter")
-    ref, mod = oracle.ref_module(fl), pkg.flavour(fl)
+    ref, mod = reference(fl), pkg.flavour(fl)
     rng = np.random.default_rng(32)
     vals = [0, 1, 97, 255, 256, 65535 if fl == "bytes" else 2 ** 32 - 1]
     for _ in range(80):
@@ -198,13 +191,12 @@ def test_streaming_over_mixed_narrow_and_wide_chunks_equals_the_oracle(monkeypat
         assert got == want, (keys, chunks)
 
 
-@needs_ref
 @pytest.mark.parametrize("fl", ["bytes", "unicode"])
-def test_ignore_white_space_uses_the_c_library_classes(fl, monkeypatch):
+def test_ignore_white_space_uses_the_c_library_classes(fl, monkeypatch, reference):
     """which letters count as white space is libc's business (iswspace / isspace, src/AutomatonSearchIter.c:265-270):
     control characters, NEL, no-break space, and for the unicode build the wide ones"""
     emul.install(monkeypatch, "filter")
-    ref, mod = oracle.ref_module(fl), pkg.flavour(fl)
+    ref, mod = reference(fl), pkg.flavour(fl)
     rng = np.random.default_rng(9)
     ws = [" ", "\t", "\n", "\x0b", "\x0c", "\r", "\x85", "\xa0", "\x1c", "\x1f"]
     if fl == "unicode":
@@ -216,7 +208,7 @@ def test_ignore_white_space_uses_the_c_library_classes(fl, monkeypatch):
         return s.encode("latin-1") if fl == "bytes" else s
 
     for _ in range(150):
-        keys = list({word(1, 5, list("ab")) for _ in range(int(rng.integers(1, 6)))})
+        keys = list(dict.fromkeys(word(1, 5, list("ab")) for _ in range(int(rng.integers(1, 6)))))
         A, R = mod.Automaton(), ref.Automaton()
         for i, k in enumerate(keys):
             A.add_word(k, i), R.add_word(k, i)
@@ -225,13 +217,12 @@ def test_ignore_white_space_uses_the_c_library_classes(fl, monkeypatch):
         assert list(A.iter(hay, ignore_white_space=True)) == list(R.iter(hay, ignore_white_space=True)), (keys, hay)
 
 
-@needs_ref
 @pytest.mark.parametrize("fl", ["bytes", "unicode"])
-def test_searches_between_random_mutations(fl, monkeypatch):
+def test_searches_between_random_mutations(fl, monkeypatch, reference):
     """add_word / remove_word / make_automaton in random order, searching whenever the reference can (and raising
     like it when it cannot) -- including automata from which every key has been removed again"""
     emul.install(monkeypatch, "filter")
-    ref, mod = oracle.ref_module(fl), pkg.flavour(fl)
+    ref, mod = reference(fl), pkg.flavour(fl)
     rng = np.random.default_rng(13)
     al = "abc" if fl == "bytes" else "abł"
 
@@ -268,13 +259,12 @@ def test_searches_between_random_mutations(fl, monkeypatch):
         assert len(A) == len(R) and A.kind == R.kind
 
 
-@needs_ref
 @pytest.mark.parametrize("fl", ["bytes", "unicode"])
-def test_iter_long_ranges_and_batch(fl, monkeypatch):
+def test_iter_long_ranges_and_batch(fl, monkeypatch, reference):
     """iter_long(string, [start, [end]]) uses find_all's range rules (src/Automaton.c:968-1040); find_long_batch ==
     looping it.  The unicode key sets mix latin-1 and other letters over latin-1 haystacks on purpose."""
     emul.install(monkeypatch, "filter")
-    ref, mod = oracle.ref_module(fl), pkg.flavour(fl)
+    ref, mod = reference(fl), pkg.flavour(fl)
     rng = np.random.default_rng(17)
     al = "abc" if fl == "bytes" else "abł"
 
@@ -283,7 +273,7 @@ def test_iter_long_ranges_and_batch(fl, monkeypatch):
         return s.encode() if fl == "bytes" else s
 
     for _ in range(120):
-        keys = list({word(1, 6) for _ in range(int(rng.integers(1, 8)))})
+        keys = list(dict.fromkeys(word(1, 6) for _ in range(int(rng.integers(1, 8)))))
         A, R = mod.Automaton(), ref.Automaton()
         for i, k in enumerate(keys):
             A.add_word(k, i), R.add_word(k, i)

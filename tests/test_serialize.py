@@ -2,7 +2,8 @@
 
 * golden: tests/golden/golden_serialized.json holds what the UNMODIFIED reference wrote
   (tests/golden/make_serialized.py); the drop-in must read it and answer like the reference did.
-* differential (needs oracle/_ref): what the drop-in writes, the reference must read; random key sets.
+* differential (the reference as recorded in tests/golden/reference): what the drop-in writes, the reference must
+  read; random key sets.
 * malformed input is refused with the reference's exception types, never a crash.
 """
 import base64
@@ -14,9 +15,9 @@ import struct
 import numpy as np
 import pytest
 
-import oracle
 import pyahocorasick_b200 as pkg
 from pyahocorasick_b200 import serialize
+from recorded_reference import reference  # noqa: F401 -- fixture
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 GOLD = json.load(open(os.path.join(HERE, "golden", "golden_serialized.json")))
@@ -67,8 +68,7 @@ def test_reads_what_the_reference_wrote(idx, tmp_path, monkeypatch):
             assert [[e, json.dumps(v)] for e, v in X.iter(hay)] == sc["iter"]
 
 
-def _build_pair(fl, store, words, rng):
-    ref = oracle.ref_module(fl)
+def _build_pair(ref, fl, store, words, rng):
     mod = pkg.flavour(fl)
     A, R = mod.Automaton(store), ref.Automaton(store)
     for i, w in enumerate(words):
@@ -86,19 +86,18 @@ def _build_pair(fl, store, words, rng):
 def _random_words(fl, rng, n):
     if fl == "bytes":
         al = np.frombuffer(b"abc\x80\xfe\xff", dtype=np.uint8)
-        return list({bytes(al[rng.integers(0, len(al), size=int(rng.integers(1, 7)))].tolist()) for _ in range(n)})
+        return list(dict.fromkeys(bytes(al[rng.integers(0, len(al), size=int(rng.integers(1, 7)))].tolist()) for _ in range(n)))
     al = "ab\xe9\u0142\U0001f600\uffff"
-    return list({"".join(al[int(j)] for j in rng.integers(0, len(al), size=int(rng.integers(1, 7)))) for _ in range(n)})
+    return list(dict.fromkeys("".join(al[int(j)] for j in rng.integers(0, len(al), size=int(rng.integers(1, 7)))) for _ in range(n)))
 
 
-@pytest.mark.skipif(not oracle.ref_available("bytes"), reason="needs oracle/_ref (built where /root/reference exists)")
 @pytest.mark.parametrize("fl", ["bytes", "unicode"])
 @pytest.mark.parametrize("store", [30, 20, 10])
-def test_the_reference_reads_what_we_write(fl, store, tmp_path):
+def test_the_reference_reads_what_we_write(fl, store, tmp_path, reference):
     rng = np.random.default_rng(1234 + store)
     for rnd in range(4):
         words = _random_words(fl, rng, 40)
-        mod, ref, A, R = _build_pair(fl, store, words, rng)
+        mod, ref, A, R = _build_pair(reference(fl), fl, store, words, rng)
         if rnd & 1:
             for w in words[::5]:
                 assert A.remove_word(w) and R.remove_word(w)
@@ -159,7 +158,7 @@ def test_key_sequence_and_empty_round_trips(tmp_path):
         assert mod.load(pe, pickle.loads).kind == mod.EMPTY
 
 
-def test_large_automaton_is_split_into_16MB_arrays_like_the_reference():
+def test_large_automaton_is_split_into_16MB_arrays_like_the_reference(reference):
     mod = pkg.flavour("bytes")
     rng = np.random.default_rng(5)
     A = mod.Automaton(mod.STORE_LENGTH)
@@ -173,9 +172,8 @@ def test_large_automaton_is_split_into_16MB_arrays_like_the_reference():
     B = mod.Automaton(*args)
     assert len(B) == len(A) and B.get_stats()["nodes_count"] == A.get_stats()["nodes_count"]
     assert all(B.get(row.tobytes()) == 12 for row in raw[::997])
-    if oracle.ref_available("bytes"):
-        R = oracle.ref_module("bytes").Automaton(*args)
-        assert len(R) == len(A) and all(R.get(row.tobytes()) == 12 for row in raw[::997])
+    R = reference("bytes").Automaton(*args)
+    assert len(R) == len(A) and all(R.get(row.tobytes()) == 12 for row in raw[::997])
 
 
 def test_argument_rules_and_malformed_input(tmp_path):
